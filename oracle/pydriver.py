@@ -44,6 +44,16 @@ def available(kind: str, fast: bool = False) -> bool:
     return os.path.exists(lib_path(kind, fast))
 
 
+def reference_source():
+    """The reference source tree oracle/_ref was compiled from (`make ref` records it), or None where it is absent."""
+    p = os.path.join(HERE, "_ref", "source_dir")
+    if not os.path.exists(p):
+        return None
+    with open(p) as fh:
+        d = fh.read().strip()
+    return d if os.path.isdir(os.path.join(d, "src", "lib")) else None
+
+
 _cache = {}
 
 

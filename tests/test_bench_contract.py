@@ -37,8 +37,11 @@ def test_reference_arm_prints_one_contract_line(build_libs):
     assert d["vs_baseline"] is None and d["data"] == "synthetic"
     assert "workload" in d["config"] and "model" not in d["config"]
     assert d["value"] > 0 and abs(d["ms_per_step"] * d["value"] - 1000.0) < 1.0
+    from oracle import pydriver
     cb = d["cpu_baseline"]
-    assert cb["kind"] == "reference" and cb["cores"] >= 1 and cb["value"] == d["value"] and cb["sample"]
+    # the compiled reference when oracle/_ref was built from its sources, else the restatement ("port") stands in
+    assert cb["kind"] == ("reference" if pydriver.available("reference", fast=True) else "port")
+    assert cb["cores"] >= 1 and cb["value"] == d["value"] and cb["sample"]
     e2e = d["e2e"]
     assert e2e["value"] == d["value"] and e2e["unit"] == d["unit"]
     assert e2e["h2d_bytes_per_step"] == 0 and e2e["d2h_bytes_per_step"] == 0

@@ -691,7 +691,7 @@ def test_nccl_sharded_pipeline_two_gpus(tmp_path):
     import sys
     import torch
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (run under gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     root = os.path.dirname(HERE)
     r = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node=2",
                         "--master-addr", "127.0.0.1", "--master-port", "29517", os.path.join(root, "tools", "run_sharded.py"),
@@ -706,7 +706,7 @@ def test_cube_sharded_pipeline_two_gpus(tmp_path):
     import sys
     import torch
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (run under gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     root = os.path.dirname(HERE)
     r = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node=2",
                         "--master-addr", "127.0.0.1", "--master-port", "29519", os.path.join(root, "tools", "run_sharded.py"),

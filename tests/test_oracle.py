@@ -1,5 +1,6 @@
 """CPU-only checks of the checker itself: the restatement against the golden vectors recorded from the compiled
-reference, against the compiled reference live (when present), and its pieces against independent numpy answers."""
+reference (tests/golden/make_golden.py), and its pieces against independent numpy answers."""
+import hashlib
 import math
 import os
 
@@ -7,6 +8,31 @@ import numpy as np
 import pytest
 
 HERE = os.path.dirname(os.path.abspath(__file__))
+
+
+def _golden(name):
+    return np.load(os.path.join(HERE, "golden", name))
+
+
+def _sha256(a):
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+def assert_input(a, g, key):
+    """The generator reproduced the input the golden run was recorded on."""
+    assert _sha256(a) == str(g[key + "__sha256"]), f"{key}: synth no longer generates the recorded input"
+
+
+def assert_golden(got, g, key):
+    """Bit-exact comparison with a recorded array, stored whole or as SHA-256 + shape + evenly spaced sample rows."""
+    if key in g.files:
+        np.testing.assert_array_equal(got, g[key], err_msg=key)
+        return
+    got = np.ascontiguousarray(got)
+    assert got.shape == tuple(g[key + "__shape"]), (key, got.shape, tuple(g[key + "__shape"]))
+    rows = np.unique(np.linspace(0, got.shape[0] - 1, 16).astype(np.int64))
+    np.testing.assert_array_equal(got[rows], g[key + "__sample"], err_msg=key)
+    assert _sha256(got) == str(g[key + "__sha256"]), key
 
 
 @pytest.fixture(scope="module")
@@ -52,24 +78,28 @@ def test_restatement_pieces_match_golden(oracle, golden_pieces):
     np.testing.assert_array_equal(oracle.lsq53(g["P5"]), g["x53"])
 
 
-def test_restatement_equals_compiled_reference_live(oracle, reference, scene):
-    """Full pipeline, bit for bit, on sweeps the fixtures do not contain (only where oracle/_ref exists)."""
+def test_restatement_equals_compiled_reference_live(oracle, scene):
+    """Full pipeline, bit for bit, against the compiled reference's run on a second trajectory (60 k map, VLP-16 at 900
+    azimuth steps, backwards yaw, sideways drift) recorded in golden/pipeline_vlp16_900_live.npz."""
     from loam_velodyne_b200 import synth
+    g = _golden("pipeline_vlp16_900_live.npz")
     lidar = synth.Lidar(16, 900, -15.0, 15.0)
     corner, surf = synth.make_map(scene, 60_000)
-    pr, po = reference.pipeline(), oracle.pipeline()
-    pr.seed_map(corner, surf)
+    assert_input(corner, g, "map_corner")
+    assert_input(surf, g, "map_surf")
+    po = oracle.pipeline()
     po.seed_map(corner, surf)
     for i in range(5):
         pts, rs = synth.make_sweep(scene, lidar, 20 + i, yaw_rate=math.radians(-7.0), v=(0.3, 0.0, 1.5))
-        _, od_r, aft_r, _ = pr.sweep(pts, rs)
-        _, od_o, aft_o, _ = po.sweep(pts, rs)
-        np.testing.assert_array_equal(od_r, od_o)
-        np.testing.assert_array_equal(aft_r, aft_o)
+        assert_input(pts, g, f"pts{i}")
+        ok_o, od_o, aft_o, _ = po.sweep(pts, rs)
+        assert ok_o == bool(g[f"ok{i}"])
+        np.testing.assert_array_equal(od_o, g[f"odom{i}"])
+        np.testing.assert_array_equal(aft_o, g[f"aft{i}"])
         for name in ("sharp", "less_sharp", "flat", "less_flat"):
-            np.testing.assert_array_equal(pr.scanreg.cloud(name), po.scanreg.cloud(name))
+            assert_golden(po.scanreg.cloud(name), g, f"{name}{i}")
         for name in ("last_corner", "last_surf"):
-            np.testing.assert_array_equal(pr.odom.cloud(name), po.odom.cloud(name))
+            assert_golden(po.odom.cloud(name), g, f"{name}{i}")
 
 
 VARIANTS = {
@@ -83,31 +113,34 @@ VARIANTS = {
 
 
 @pytest.mark.parametrize("variant", sorted(VARIANTS))
-def test_restatement_equals_compiled_reference_variants(oracle, reference, scene, variant):
+def test_restatement_equals_compiled_reference_variants(oracle, scene, variant):
     """Other sensor geometries, ragged rings (returns beyond max range dropped), non-default RegistrationParams and tight
-    iteration budgets: the restatement and the compiled reference agree bit for bit on poses, features and map."""
+    iteration budgets: the restatement agrees bit for bit on poses, features and map with the compiled reference's run
+    recorded in golden/pipeline_variants.npz."""
     from loam_velodyne_b200 import synth
+    g = _golden("pipeline_variants.npz")
     R, A, lo, hi, yaw, v, max_range, reg, (oi, mi) = VARIANTS[variant]
     lidar = synth.Lidar(R, A, lo, hi)
     corner, surf = synth.make_map(scene, 40_000)
-    pr, po = reference.pipeline(odom_iter=oi, map_iter=mi), oracle.pipeline(odom_iter=oi, map_iter=mi)
-    for p in (pr, po):
-        if reg:
-            p.scanreg.configure(**reg)
-        p.seed_map(corner, surf)
+    assert_input(corner, g, "map_corner")
+    assert_input(surf, g, "map_surf")
+    po = oracle.pipeline(odom_iter=oi, map_iter=mi)
+    if reg:
+        po.scanreg.configure(**reg)
+    po.seed_map(corner, surf)
     for i in range(4):
         pts, rs = synth.make_sweep(scene, lidar, 5 + i, yaw_rate=math.radians(yaw), v=v, max_range=max_range)
+        assert_input(pts, g, f"{variant}/pts{i}")
         if max_range > 0:
             assert len(set(rs.tolist())) > 1  # the rings really are ragged
-        ok_r, od_r, aft_r, _ = pr.sweep(pts, rs)
         ok_o, od_o, aft_o, _ = po.sweep(pts, rs)
-        assert ok_r == ok_o
-        np.testing.assert_array_equal(od_r, od_o)
-        np.testing.assert_array_equal(aft_r, aft_o)
+        assert ok_o == bool(g[f"{variant}/ok{i}"])
+        np.testing.assert_array_equal(od_o, g[f"{variant}/odom{i}"])
+        np.testing.assert_array_equal(aft_o, g[f"{variant}/aft{i}"])
         for name in ("sharp", "less_sharp", "flat", "less_flat"):
-            np.testing.assert_array_equal(pr.scanreg.cloud(name), po.scanreg.cloud(name))
-    np.testing.assert_array_equal(pr.mapping.cloud("corner_cubes"), po.mapping.cloud("corner_cubes"))
-    np.testing.assert_array_equal(pr.mapping.cloud("surf_cubes"), po.mapping.cloud("surf_cubes"))
+            assert_golden(po.scanreg.cloud(name), g, f"{variant}/{name}{i}")
+    assert_golden(po.mapping.cloud("corner_cubes"), g, f"{variant}/corner_cubes")
+    assert_golden(po.mapping.cloud("surf_cubes"), g, f"{variant}/surf_cubes")
 
 
 def test_knn_against_brute_force(oracle):
@@ -180,21 +213,24 @@ def test_feature_edge_cases_do_not_crash(oracle):
     assert s.cloud("sharp").shape[0] <= 12 * len(sizes)
 
 
-def test_ring_binning_restatement_equals_compiled_reference(oracle, reference, scene):
-    """MultiScanRegistration::process (unmodified reference adapter compiled against oracle/shim/ros) vs the CPU
-    restatement: binned cloud, ring sizes and the extracted features are bit-identical."""
+def test_ring_binning_restatement_equals_compiled_reference(oracle, scene):
+    """MultiScanRegistration::process (unmodified reference adapter compiled against oracle/shim/ros, recorded in
+    golden/multiscan_vlp16_hdl64.npz) vs the CPU restatement: binned cloud, ring sizes and the extracted features are
+    bit-identical."""
     from loam_velodyne_b200 import synth
-    for lidar, bounds, jitter in ((synth.Lidar.vlp16(), (-15.0, 15.0, 16), 0.0), (synth.Lidar.hdl64(), (-24.9, 2.0, 64), 0.15)):
+    g = _golden("multiscan_vlp16_hdl64.npz")
+    for key, lidar, bounds, jitter in (("vlp16", synth.Lidar.vlp16(), (-15.0, 15.0, 16), 0.0),
+                                       ("hdl64", synth.Lidar.hdl64(), (-24.9, 2.0, 64), 0.15)):
         pts, rs = synth.make_sweep(scene, lidar, 2, yaw_rate=math.radians(5.0))
         raw = synth.raw_cloud_from_sweep(pts, rs, n_bad=37, seed=5, elev_jitter_deg=jitter)
-        a, b = oracle.multiscan(*bounds), reference.multiscan(*bounds)
+        assert_input(raw, g, f"{key}/raw")
+        a = oracle.multiscan(*bounds)
         pa, sa = a.process(raw)
-        pb, sb = b.process(raw)
-        np.testing.assert_array_equal(sa, sb)
-        np.testing.assert_array_equal(pa, pb)
+        np.testing.assert_array_equal(sa, g[f"{key}/sizes"])
+        assert_golden(pa, g, f"{key}/binned")
         assert pa.shape[0] > 0.9 * pts.shape[0]
         for name in ("sharp", "less_sharp", "flat", "less_flat"):
-            np.testing.assert_array_equal(a.cloud(name), b.cloud(name))
+            assert_golden(a.cloud(name), g, f"{key}/{name}")
         if jitter == 0.0:
             # exact ring geometry: every point returns to the ring it was cast from, in firing order
             np.testing.assert_array_equal(sa, rs)
@@ -212,19 +248,25 @@ def test_ring_binning_restatement_matches_golden(oracle):
     np.testing.assert_array_equal(ms.cloud("flat"), g["flat"])
 
 
-def test_transform_maintenance(oracle, reference):
-    """BasicTransformMaintenance: restatement == compiled reference == the library's drop-in class, bit for bit
-    (host-only arithmetic; the drop-in shares its association routine with BasicLaserMapping's pose prediction)."""
+def test_transform_maintenance(oracle):
+    """BasicTransformMaintenance: restatement == compiled reference (golden/transform_maintenance.npz) == the library's
+    drop-in class, bit for bit (host-only arithmetic; the drop-in shares its association routine with
+    BasicLaserMapping's pose prediction)."""
     from loam_velodyne_b200 import api
+    g = _golden("transform_maintenance.npz")
     rng = np.random.RandomState(21)
-    for _ in range(200):
+    inputs = []
+    for k in range(200):
         sum6 = np.concatenate([rng.uniform(-0.6, 0.6, 3), rng.uniform(-40, 40, 3)]).astype(np.float32)
         bef6 = (sum6 + np.concatenate([rng.normal(0, 0.02, 3), rng.normal(0, 0.5, 3)])).astype(np.float32)
         aft6 = (bef6 + np.concatenate([rng.normal(0, 0.01, 3), rng.normal(0, 0.2, 3)])).astype(np.float32)
-        r = reference.transform_maintenance(sum6, bef6, aft6)
+        inputs.append(np.stack([sum6, bef6, aft6]))
+        r = g["mapped"][k]
         np.testing.assert_array_equal(oracle.transform_maintenance(sum6, bef6, aft6), r)
         np.testing.assert_array_equal(api.transform_maintenance(sum6, bef6, aft6), r)
         assert np.isfinite(r).all()
+    assert_input(np.stack(inputs), g, "inputs")
     # identity correction: mapped == odometry pose
     p = np.array([0.1, -0.2, 0.05, 1.0, 2.0, 3.0], np.float32)
-    np.testing.assert_allclose(reference.transform_maintenance(p, p, p), p, rtol=0, atol=2e-6)
+    np.testing.assert_allclose(g["identity_out"], p, rtol=0, atol=2e-6)
+    np.testing.assert_array_equal(oracle.transform_maintenance(p, p, p), g["identity_out"])
