@@ -320,6 +320,8 @@ struct loam_b200_ctx {
   } store[2];
   bool map_use_store = false;      // scan-to-map search goes through the store (stage API) / through grid[] (kernel API)
   bool map_debug_from_map = false; // begin_sweep also materialises the from-map clouds (tests)
+  bool split_map_update = false;   // every end-of-sweep update takes the multi-launch chain (LOAM_B200_SPLIT_MAP_UPDATE
+                                   // at creation; the reference the single-cluster chain is tested against)
   loamb::DevBuf<float4> pool_tmp;
   loamb::DevBuf<unsigned char> pool_tmp_cls;
   loamb::DevBuf<unsigned> cmp_pos, cmp_bsum;

@@ -609,7 +609,10 @@ int loam_b200_create(loam_b200_ctx** out, int device) {
     cudaFuncSetAttribute(voxel_filter_cluster_kernel<false>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
     cudaFuncSetAttribute(bvh_build_cluster_kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
     cudaFuncSetAttribute(cluster_sort_pairs_kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
+    cudaFuncSetAttribute(store_front_cluster_kernel<true>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
+    cudaFuncSetAttribute(store_front_cluster_kernel<false>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
   }
+  c->split_map_update = getenv("LOAM_B200_SPLIT_MAP_UPDATE") != nullptr;
   c->cluster_ok = !getenv("LOAM_B200_NO_CLUSTER") &&
                   cudaFuncSetAttribute(voxel_filter_cluster_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                        (int)sizeof(ClusterSortSmem)) == cudaSuccess &&
@@ -618,6 +621,10 @@ int loam_b200_create(loam_b200_ctx** out, int device) {
                   cudaFuncSetAttribute(bvh_build_cluster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                        (int)sizeof(ClusterSortSmem)) == cudaSuccess &&
                   cudaFuncSetAttribute(cluster_sort_pairs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       (int)sizeof(ClusterSortSmem)) == cudaSuccess &&
+                  cudaFuncSetAttribute(store_front_cluster_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       (int)sizeof(ClusterSortSmem)) == cudaSuccess &&
+                  cudaFuncSetAttribute(store_front_cluster_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                        (int)sizeof(ClusterSortSmem)) == cudaSuccess;
   cudaGetLastError();
   if (c->partials.reserve(4096 * NEQ) != cudaSuccess || c->result.reserve(NEQ) != cudaSuccess ||

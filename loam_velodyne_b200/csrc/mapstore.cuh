@@ -18,6 +18,7 @@
 // stay unfiltered, exactly like the reference's cube clouds, until their cube is visible at the end of a sweep.
 #pragma once
 
+#include "clustersort.cuh"
 #include "gridnn.cuh"
 #include "mappool.cuh"
 
@@ -259,18 +260,106 @@ __global__ void store_raw_select_scatter_kernel(const float4* __restrict__ pool,
   vals[d] = d;
 }
 
+// Front of the end-of-sweep update in ONE cluster launch (S <= CS_MAX_N): [INSERT: store_insert_kernel's points and
+// filter keys of the stack] -> stable sort by filter key (cluster_sort, radix_sort_pairs' four passes) -> voxel run
+// heads.  It leaves what the multi-launch front (store_insert_kernel, radix_sort_pairs, voxel_head_kernel +
+// radix_scan_kernel) leaves for store_voxel_merge_kernel: the sorted (key, index) pairs in place over keys / vals, and
+// pos[i] = heads before i | head flag << 31, here as global ranks with block_off[0..nb] = 0.  Without INSERT the
+// unsorted S is read from keys / vals (raw seed points joined it, store_raw_select_scatter_kernel).
+template <bool INSERT>
+__global__ void __cluster_dims__(CS_CL, 1, 1) __launch_bounds__(CS_THREADS)
+store_front_cluster_kernel(const float4* __restrict__ stack_ds, int n, MapIterArgs a, CubeGrid g,
+                           const unsigned char* __restrict__ rank_of_cube, float inv_leaf, ShardSpec sh,
+                           float4* __restrict__ s_pts, unsigned* keys, int* vals, unsigned* __restrict__ pos,
+                           unsigned* __restrict__ block_off) {
+  extern __shared__ __align__(16) unsigned char cs_raw[];
+  ClusterSortSmem& sm = *reinterpret_cast<ClusterSortSmem*>(cs_raw);
+  cg::cluster_group cluster = cg::this_cluster();
+  const unsigned my = cluster.block_rank();
+  const int per = (n + CS_CL - 1) / CS_CL;
+  const int m_local = cs_local_count(n, per, my);
+  const int g0 = (int)my * per;
+  for (int i = threadIdx.x; i < m_local; i += CS_THREADS) {
+    const int gi = g0 + i;
+    if (INSERT) {
+      const float4 q = stack_ds[gi];
+      float x, y, z;
+      associate_to_map(a, q, x, y, z);
+      const float4 p = make_float4(x, y, z, q.w);
+      s_pts[gi] = p;
+      sm.keys[0][i] = shard_stores(sh, store_cell(p.x)) ? filter_key_of(p, gi, g, rank_of_cube, inv_leaf)
+                                                        : (((unsigned)CLS_DROP << 24) | ((unsigned)gi & 0xffffffu));
+      sm.vals[0][i] = gi;
+    } else {
+      sm.keys[0][i] = keys[gi];
+      sm.vals[0][i] = vals[gi];
+    }
+  }
+  if (my == 0)
+    for (int b = threadIdx.x; b <= (n + SCAN_BS - 1) / SCAN_BS; b += CS_THREADS) block_off[b] = 0;
+  __syncthreads();
+  const int cur = cluster_sort(sm, n, per, 4);
+
+  // heads before every element inside this CTA (block scan in rounds, as voxel_filter_cluster_kernel), kept in the
+  // sort's spare value buffer with the head flag in bit 31 -> exchange the CTA totals -> global ranks
+  auto key_at = [&](int gi) -> unsigned {
+    const int r = gi / per;
+    return cluster.map_shared_rank(&sm.keys[cur][0], r)[gi - r * per];
+  };
+  unsigned* rank_in_cta = reinterpret_cast<unsigned*>(&sm.vals[cur ^ 1][0]);
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  unsigned carry = 0;
+  for (int base = 0; base < m_local; base += CS_THREADS) {
+    const int i = base + threadIdx.x;
+    const bool head = i < m_local && (g0 + i == 0 || sm.keys[cur][i] != (i > 0 ? sm.keys[cur][i - 1] : key_at(g0 - 1)));
+    const unsigned bal = __ballot_sync(0xffffffffu, head);
+    if (lane == 0) sm.wsum[warp] = __popc(bal);
+    __syncthreads();
+    unsigned woff = 0, round_total = 0;
+    for (int w = 0; w < CS_NW; w++) {
+      const unsigned c = sm.wsum[w];
+      if (w < warp) woff += c;
+      round_total += c;
+    }
+    if (i < m_local) rank_in_cta[i] = (carry + woff + __popc(bal & ((1u << lane) - 1u))) | (head ? 1u << 31 : 0u);
+    carry += round_total;
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) sm.scal[0] = carry;
+  cluster.sync();
+  unsigned cta_base = 0;
+  for (unsigned r = 0; r < my; r++) cta_base += cluster.map_shared_rank(&sm.scal[0], r)[0];
+  for (int i = threadIdx.x; i < m_local; i += CS_THREADS) {
+    keys[g0 + i] = sm.keys[cur][i];
+    vals[g0 + i] = sm.vals[cur][i];
+    pos[g0 + i] = rank_in_cta[i] + cta_base;
+  }
+  cluster.sync();  // nobody leaves while a neighbour may still read its shared memory
+}
+
 // One thread per voxel run of the sorted S.  Visible voxel: centroid over [the filtered map points already in that
 // voxel (found through the cell table, marked DEAD), then the run's points in sorted order] -> one filtered point.
 // Invisible cube: the (single) point goes to the map unfiltered.  Every emitted point also gets its cell key.
+// n_runs_out (optional): the number of runs that are emitted (runs outside the grid, class 0xFF, sort last and are cut
+// off), written by the last element below them -- what runs_below_kernel computes, without a launch of its own.
 __global__ void store_voxel_merge_kernel(const float4* __restrict__ s_pts, const unsigned* __restrict__ s_keys,
                                          const int* __restrict__ s_vals, const unsigned* __restrict__ pos,
                                          const unsigned* __restrict__ block_off, int n_s, MapGridView pool,
                                          unsigned char* __restrict__ pool_state, float inv_leaf, float leaf,
                                          float4* __restrict__ e_pts, unsigned char* __restrict__ e_state,
-                                         unsigned* __restrict__ e_keys, int* __restrict__ e_vals) {
+                                         unsigned* __restrict__ e_keys, int* __restrict__ e_vals,
+                                         int* __restrict__ n_runs_out = nullptr) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n_s) return;
   const unsigned pv = pos[i];
+  if (n_runs_out) {
+    constexpr unsigned CUT = (unsigned)CLS_DROP << 24;
+    const unsigned ki = s_keys[i];
+    if (ki < CUT && (i + 1 == n_s || s_keys[i + 1] >= CUT))
+      *n_runs_out = (int)((pv & 0x7fffffffu) + block_off[i / SCAN_BS] + (pv >> 31));
+    else if (i == 0 && ki >= CUT)
+      *n_runs_out = 0;
+  }
   if (!(pv >> 31)) return;
   const unsigned dst = (pv & 0x7fffffffu) + block_off[i / SCAN_BS];
   const unsigned k = s_keys[i];
@@ -345,13 +434,27 @@ __global__ void store_voxel_merge_kernel(const float4* __restrict__ s_pts, const
   e_vals[dst] = (int)dst;
 }
 
+// what store_index_kernel fills in: cleared by the pass before the merge instead of by memsets of their own
+struct IndexClear {
+  uint4* table = nullptr;
+  unsigned table_n = 0;
+  int* stats = nullptr;  // cube_stats, 3 x CUBE_NUM
+  int* n_cells = nullptr;
+};
+
 // pool elements that survive the sweep: not replaced, and (after a roll of the grid) still inside it
 template <bool CHECK_GRID>
 __global__ void __launch_bounds__(SCAN_BS)
 store_live_count_kernel(const float4* __restrict__ pts, const unsigned char* __restrict__ st, int n,
                         const int* __restrict__ n_dev, CubeGrid g, unsigned* __restrict__ local_pos,
-                        unsigned* __restrict__ block_sums) {
+                        unsigned* __restrict__ block_sums, IndexClear clr = IndexClear{}) {
   __shared__ unsigned ws[32];
+  if (clr.table) {  // (the voxel merge, the last reader of the old table, ran before this kernel)
+    const unsigned t = blockIdx.x * SCAN_BS + threadIdx.x, stride = gridDim.x * SCAN_BS;
+    for (unsigned j = t; j < clr.table_n; j += stride) clr.table[j] = make_uint4(0u, 0u, 0u, 0u);
+    for (unsigned j = t; j < 3u * CUBE_NUM; j += stride) clr.stats[j] = 0;
+    if (t == 0) *clr.n_cells = 0;
+  }
   if (n_dev) n = min(n, *n_dev);
   const int i = blockIdx.x * SCAN_BS + threadIdx.x;
   bool live = i < n && !(st[i] & ST_DEAD);
@@ -443,6 +546,42 @@ store_merge_kernel(const float4* __restrict__ p_pts, const unsigned* __restrict_
     o_pts[dst] = e_pts[src];
     o_keys[dst] = key;
     o_state[dst] = e_state[src];
+  }
+}
+
+// grid_insert_kernel and store_stats_kernel over the merged pool in one pass: cell table entries (linear probing),
+// occupied cells -> *n_cells, per cube slot [start, end) and raw count.  Table, stats and *n_cells start zeroed.
+__global__ void store_index_kernel(const unsigned* __restrict__ keys, const unsigned char* __restrict__ st, int n,
+                                   const int* __restrict__ n_dev, uint4* __restrict__ table, unsigned mask,
+                                   int* __restrict__ n_cells, int* __restrict__ cube_start, int* __restrict__ cube_end,
+                                   int* __restrict__ cube_raw) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (n_dev) n = min(n, *n_dev);
+  const bool in = i < n;
+  const unsigned k = in ? keys[i] : 0u;
+  const unsigned slot = in ? (k >> 17) : 0xffffffffu;
+  const bool head = in && (i == 0 || keys[i - 1] != k);
+  if (in) {
+    if (i == 0 || (keys[i - 1] >> 17) != slot) cube_start[slot] = i;
+    if (i == n - 1 || (keys[i + 1] >> 17) != slot) cube_end[slot] = i + 1;
+  }
+  const bool raw = in && (st[i] & ST_RAW);
+  const unsigned peers = __match_any_sync(0xffffffffu, raw ? slot : 0xfffffffeu);
+  if (raw && (peers & ((1u << (threadIdx.x & 31)) - 1u)) == 0) atomicAdd(&cube_raw[slot], __popc(peers));
+  const int heads = __syncthreads_count(head ? 1 : 0);
+  if (threadIdx.x == 0 && heads > 0) atomicAdd(n_cells, heads);
+  if (!head) return;
+  int cnt = 1;
+  while (i + cnt < n && keys[i + cnt] == k) cnt++;
+  unsigned h = grid_hash(k) & mask;
+  for (unsigned tries = 0; tries <= mask; tries++) {  // bounded, as in grid_insert_kernel
+    const unsigned prev = atomicCAS(&table[h].x, 0u, k + 1u);
+    if (prev == 0u) {
+      table[h].y = (unsigned)i;
+      table[h].z = (unsigned)cnt;
+      return;
+    }
+    h = (h + 1) & mask;
   }
 }
 
